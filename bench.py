@@ -209,6 +209,14 @@ def run_cpu(steps, warmup, budget_s, threads=None):
     return best
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each device tensor of `arrays` as out_dir/<name>.npy in float32 (flag bytes are exact in float32)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy().astype(np.float32))
+
+
 def cpu_sample(fn, units_per_call, cores, seconds=2.5, min_calls=2):
     """units/s of `fn` on the oracle with `cores` threads, for about `seconds` of CPU work."""
     from oracle import oracle as orc_mod
@@ -592,7 +600,12 @@ def main():
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='launch every tick from Python instead of replaying a CUDA graph')
     ap.add_argument('--no-sections', action='store_true', help='skip the extra sections (stage2 / circle / sweep / train / learner)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="after the timed ticks, write what the last one returned (rank 0's agents) as DIR/<name>.npy: "
+                         'obs, reward, flags, goal_speed, eplog, pose')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get('RANK', '0'))
@@ -697,6 +710,11 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the last timed tick wrote its scans into the ring slot of its index within the graph (or the loop)
+        last = ((G if graph is not None else args.steps) - 1) % 128
+        dump_outputs(args.dump_outputs, {'obs': ring[last], 'reward': env.reward, 'flags': env.flags,
+                                         'goal_speed': env.gs, 'eplog': env.eplog, 'pose': env.state['pose']})
 
     # ---- e2e: the host-buffer call (pinned action H2D, tick, obs/reward/flags/gs D2H, sync inside every call)
     a_host = [torch.from_numpy(random_actions(rng, N)).pin_memory() for _ in range(8)]

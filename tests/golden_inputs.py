@@ -1,5 +1,7 @@
 """Deterministic synthetic weights / batches shared by tools/make_golden.py (reference side) and the GPU tests
 (our side).  Everything is derived from numpy RandomState streams, which are stable across numpy versions."""
+import os
+
 import numpy as np
 
 SHAPES = [
@@ -16,6 +18,14 @@ SHAPES = [
     ('crt_fc2.weight', (128, 260)), ('crt_fc2.bias', (128,)),
     ('critic.weight', (1, 128)), ('critic.bias', (1,)),
 ]
+
+
+def shipped_checkpoint(name):
+    """The reference's shipped policy/<name>.pth as shrunk by tools/make_golden_checkpoints.py: (state_dict of numpy
+    arrays with the shipped keys, order, shapes and dtypes; the reference CNNPolicy's App. C probes on those weights)."""
+    z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'checkpoints_sampled.npz'))
+    sd = {k.split(':', 1)[1]: z[k] for k in z.files if k.startswith(name + ':') and k != name + ':probe'}
+    return sd, z[name + ':probe']
 
 
 def synthetic_state_dict(seed=1234):

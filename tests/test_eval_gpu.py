@@ -1,5 +1,6 @@
 """Evaluation driver (SURVEY §8(f) rank 3): circle_test.enjoy and generate_action_no_sampling against the reference's
-semantics (/root/reference/circle_test.py:36-84, model/ppo.py:84-107) with the reference's shipped stage2.pth."""
+semantics (circle_test.py:36-84, model/ppo.py:84-107) with the reference's shipped stage2.pth (large matrices sampled,
+tests/golden/checkpoints_sampled.npz)."""
 import os
 import sys
 
@@ -7,17 +8,17 @@ import numpy as np
 import pytest
 import torch
 
+from golden_inputs import shipped_checkpoint
 from helpers import make_pair
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CKPT = os.path.join(ROOT, 'tests', 'golden', 'checkpoints', 'stage2.pth')
 
 
 def _policy(n):
     from rl_collision_avoidance_b200.model.net import CNNPolicy
     pol = CNNPolicy(frames=3, action_space=2, max_batch=n)
-    pol.load_state_dict(torch.load(CKPT, map_location='cpu'))
+    pol.load_state_dict({k: torch.from_numpy(v) for k, v in shipped_checkpoint('stage2')[0].items()})
     return pol
 
 

@@ -67,16 +67,16 @@ def test_stage2_golden_filter_is_our_filter():
 
 
 def test_reference_checkpoint_fixtures_have_the_23_tensors():
-    """tests/golden/checkpoints/*.pth are the reference's shipped policy/*.pth (data fixtures): same keys and shapes as
-    our flat parameter layout (SURVEY App. C)."""
+    """tests/golden/checkpoints_sampled.npz holds the reference's shipped policy/*.pth (data fixtures, the large
+    matrices sampled): same keys, key order and shapes as our flat parameter layout (SURVEY App. C)."""
     sys_path = os.path.dirname(__file__)
     import sys
     sys.path.insert(0, sys_path)
-    from golden_inputs import SHAPES
+    from golden_inputs import SHAPES, shipped_checkpoint
     for name in ('stage1_1', 'stage1_2', 'stage2'):
-        sd = torch.load(os.path.join(sys_path, 'golden', 'checkpoints', name + '.pth'), map_location='cpu')
+        sd, _ = shipped_checkpoint(name)
         assert [(k, tuple(v.shape)) for k, v in sd.items()] == [(k, tuple(s)) for k, s in SHAPES]
-        assert all(v.dtype == torch.float32 for v in sd.values())
+        assert all(v.dtype == np.float32 for v in sd.values())
 
 
 def test_transform_buffer_matches_reference_golden():

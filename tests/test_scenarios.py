@@ -3,7 +3,6 @@ import math
 import os
 
 import numpy as np
-import pytest
 
 from rl_collision_avoidance_b200 import _lib
 from rl_collision_avoidance_b200.scenarios import COMMON, fill_config, make_scenario
@@ -45,10 +44,12 @@ def test_fill_config_derived_fields():
     assert cfg.robots_per_world * cfg.num_worlds == 4104
 
 
-@pytest.mark.skipif(not os.path.exists('/root/reference/worlds/stage1.world'), reason='reference not mounted')
 def test_assets_reproduce_from_reference_worlds():
+    """The packaged maps are what the world loader makes of the reference's own world files and bitmaps, which are
+    stored unmodified as fixtures under tests/golden/worlds/."""
     from rl_collision_avoidance_b200.worldfile import load_world
+    worlds = os.path.join(os.path.dirname(__file__), 'golden', 'worlds')
     for name in ('stage1', 'stage2'):
-        m = load_world(f'/root/reference/worlds/{name}.world')
+        m = load_world(os.path.join(worlds, f'{name}.world'))
         a = make_scenario(name).map
         assert np.array_equal(m.cells, a.cells) and (m.origin_cx, m.origin_cy) == (a.origin_cx, a.origin_cy)

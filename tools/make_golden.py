@@ -166,22 +166,6 @@ def main():
     out['ppo2_after_act_fc1.weight_rows'] = after['act_fc1.weight'].numpy()[::37, ::301]
     out['ppo2_after_crt_fc1.weight_rows'] = after['crt_fc1.weight'].numpy()[::41, ::307]
 
-    # ---- the reference's shipped checkpoints (policy/*.pth, loaded at ppo_stage1.py:185-191 / ppo_stage2.py:194-200 /
-    # circle_test.py:97-103): SURVEY App. C's free / ramp probes through the reference's own CNNPolicy
-    free_obs = torch.full((1, 3, 512), 0.5)
-    ramp_obs = (torch.arange(512, dtype=torch.float32) / 511 - 0.5).view(1, 1, 512).repeat(1, 3, 1)
-    for name in ('stage1_1', 'stage1_2', 'stage2'):
-        pol = CNNPolicy(frames=3, action_space=2)
-        pol.load_state_dict(torch.load(os.path.join(REF, 'policy', name + '.pth'), map_location='cpu'))
-        with torch.no_grad():
-            v_f, _, _, m_f = pol(free_obs, torch.tensor([[5.0, 0.0]]), torch.tensor([[0.0, 0.0]]))
-            v_r, _, _, m_r = pol(ramp_obs, torch.tensor([[3.0, -1.0]]), torch.tensor([[0.5, 0.2]]))
-            _, lp, ent = pol.evaluate_actions(free_obs, torch.tensor([[5.0, 0.0]]), torch.tensor([[0.0, 0.0]]),
-                                              torch.tensor([[0.7, 0.1]]))
-        out['ckpt_' + name] = np.array([v_f.item(), m_f[0, 0].item(), m_f[0, 1].item(), v_r.item(), m_r[0, 0].item(),
-                                        m_r[0, 1].item(), lp.item(), ent.item()], np.float64)
-        print(name, out['ckpt_' + name])
-
     path = os.path.join(ROOT, 'tests', 'golden', 'learner_golden.npz')
     np.savez_compressed(path, **out)
     print('wrote', path, {k: np.asarray(v).shape for k, v in out.items() if k.startswith(('fwd', 'ppo_losses', 'loss0'))})
